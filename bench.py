@@ -1,6 +1,6 @@
 """Benchmark of the Wan DiT denoise-step hot path (BASELINE.json metric: denoise-step latency & frames/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--shape A|B] [--impl b200|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--shape A|B] [--impl b200|reference] [--no-extras] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch of synthetic input = one denoise step of the DiT block stack
@@ -19,6 +19,13 @@ literal [1,24,32760,64] SageSLA shape, LTX-2 shape C kernels), so the driver's B
 --impl reference times the reference's own CPU path for this metric: torch SDPA dense attention
 (rcm/utils/attention.py:152-166 body) on the bench's q/k/v shape, on all host cores; each step is ONE layer's attention call
 (a bounded sample: 1 of `layers` blocks, linears excluded), value scales it by the layer count only.
+
+--dump-outputs DIR writes DIR/step_output.npy after the timed steps: the output of the last timed step in float32, a fixed
+sample of its rows (output_sample).  Weights and inputs are seeded, so every run with the same arguments sees the same inputs.
+The output is not bit-reproducible: the fused attention sums its linear-attention moments with fp32 atomics in a run-dependent
+order, and 30 blocks amplify that.  In three runs of one build at shape A on one B200 (1000 W power limit), every pair of
+dumps differed by rel-L2 1.87e-2 (cos 0.99983, max |diff| <= 0.25 at max |y| 6.6; profiles/r03_dump_run_to_run.txt, which
+lists the commands).  Compare dumps of two builds with a tolerance above that spread.
 """
 from __future__ import annotations
 
@@ -43,6 +50,7 @@ SHAPES = {
     "B": dict(name="Wan2.1-T2V-14B-720p", L=75600, dim=5120, heads=40, ffn=13824, layers=40, text=512, thw=(21, 45, 80)),
 }
 FRAMES, DENOISE_STEPS = 81, 4
+DUMP_BYTES = 48 << 20  # --dump-outputs stays below 64 MB: the full step output is 200 MB (shape A) / 1.5 GB (shape B) in float32
 
 
 def peaks():
@@ -222,9 +230,26 @@ def ncu_traffic(shape_key, world):
     return {"traffic": None}
 
 
-def run_b200(shape_key, shape, args, dev, rank, world, local_rank, steps, warmup, want_e2e, sp_mode_req):
+def output_sample(y, L, row0, world):
+    """The rows of the step output [L, dim] that --dump-outputs writes, as float32 on the host: a fixed sample (randperm of
+    torch.Generator().manual_seed(0)) of at most DUMP_BYTES, in ascending row order.  Under sequence parallelism every rank
+    contributes the sampled rows of its shard [row0, row0 + local rows) and every rank returns the whole sample."""
+    import torch.distributed as dist
+    n = min(L, DUMP_BYTES // (4 * y.shape[1]))
+    rows = torch.randperm(L, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    mine = rows[(rows >= row0) & (rows < row0 + y.shape[0])] - row0
+    part = y[mine.to(y.device)].float().cpu()
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, part)   # shards are contiguous and in rank order
+        part = torch.cat(parts)
+    return part
+
+
+def run_b200(shape_key, shape, args, dev, rank, world, local_rank, steps, warmup, want_e2e, sp_mode_req, dump=False):
     """Build the block stack of `shape`, time `steps` denoise steps (eager pass with per-kernel events, then CUDA-graph
-    replay), optionally the end-to-end variant with host buffers.  Returns a dict of measurements."""
+    replay), optionally the end-to-end variant with host buffers.  Returns a dict of measurements; with `dump`, also
+    res["dump"]: output_sample() of what the timed path computed in its last step."""
     import torch.distributed as dist
     from turbodiffusion_b200 import _lib
     from turbodiffusion_b200 import turbo_diffusion_ops as tdo
@@ -326,6 +351,8 @@ def run_b200(shape_key, shape, args, dev, rank, world, local_rank, steps, warmup
            "sp_mode": sp_mode, "n_gemm": n_gemm, "gemm_ms": gemm_ms, "gemm_flops": gemm_flops, "gemm_share": gemm_ms / eager_total,
            "n_attn": n_attn, "attn_ms": attn_ms, "attn_flops": attn_flops, "attn_share": attn_ms / eager_total,
            "rows": rows}
+    if dump:
+        res["dump"] = output_sample(ys if graph is not None else y, L, row0, world)
 
     # (3) end to end through the public call with HOST buffers (H2D of the inputs + D2H of the result per step)
     if want_e2e:
@@ -470,7 +497,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra_configs runs (shape B, 24x64, LTX shape C)")
     ap.add_argument("--profile", action="store_true", help="device-resident region only (for runs under ncu)")
     ap.add_argument("--no-graph", action="store_true", help="time the eager (Python-launched) step instead of the CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output of the last timed step as DIR/step_output.npy (float32, a "
+                         "fixed sample of its rows, see output_sample) so that two builds can be compared on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the output of the b200 step; --impl reference times a CPU attention call with nothing to compare")
     if args.profile:
         args.no_graph = True
         args.no_extras = True
@@ -503,7 +537,12 @@ def main():
             print(f"[bench] gloo exit group unavailable ({type(ex).__name__}: {ex}); using the NCCL barrier", file=sys.stderr)
             exit_group = None
 
-    res = run_b200(args.shape, shape, args, dev, rank, world, local_rank, args.steps, args.warmup, not args.profile, args.sp_mode)
+    res = run_b200(args.shape, shape, args, dev, rank, world, local_rank, args.steps, args.warmup, not args.profile, args.sp_mode,
+                   dump=args.dump_outputs is not None)
+    if args.dump_outputs is not None and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "step_output.npy"), res.pop("dump").numpy())
     if args.profile:
         if rank == 0:
             print(json.dumps({"profile_run": True, "ms_per_step": res["ms_step"], "gpu_launches": res["launches"]}), flush=True)

@@ -1,5 +1,6 @@
 """Host-side pieces of bench.py that can run without a GPU: the clock sampler's windowing (against a fake nvidia-smi), the
-reference arm's JSON line (the CPU path the driver times beside the GPU arm), and the multi-rank exit path."""
+reference arm's JSON line (the CPU path timed beside the GPU arm), argument checks, the --dump-outputs row sample, and the
+multi-rank exit path."""
 import importlib.util
 import json
 import os
@@ -74,6 +75,59 @@ def test_reference_arm_prints_the_contract_line():
     assert line["cpu_baseline"]["value"] == line["value"] > 0
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0 and line["e2e"]["value"] == line["value"]
     assert line["config"]["L"] == 32760 and line["config"]["heads"] == 12
+
+
+@pytest.mark.parametrize("argv,message", [(["--steps", "0"], "--steps must be at least 1"),
+                                          (["--impl", "reference", "--dump-outputs", "unused"], "--dump-outputs writes the output of")])
+def test_bad_arguments_are_refused(argv, message):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=600,
+                         cwd=ROOT)
+    assert out.returncode == 2 and message in out.stderr
+
+
+def test_output_sample_is_a_fixed_sorted_row_sample_within_the_budget(monkeypatch):
+    import torch
+    b = _bench()
+    y = torch.arange(1000, dtype=torch.float32)[:, None].repeat(1, 8)     # every row holds its own index
+    monkeypatch.setattr(b, "DUMP_BYTES", 100 * 8 * 4)
+    s = b.output_sample(y, 1000, 0, 1)
+    assert s.dtype == torch.float32 and s.shape == (100, 8) and torch.equal(s, y[s[:, 0].long()])
+    assert (s[1:, 0] > s[:-1, 0]).all() and torch.equal(s, b.output_sample(y, 1000, 0, 1))
+    monkeypatch.setattr(b, "DUMP_BYTES", 1 << 20)                          # an output within the budget is written whole
+    assert torch.equal(b.output_sample(y, 1000, 0, 1), y)
+
+
+_SAMPLE_SCRIPT = """
+import importlib.util, os, sys
+import torch, torch.distributed as dist
+spec = importlib.util.spec_from_file_location("bench_module", sys.argv[1]); b = importlib.util.module_from_spec(spec); spec.loader.exec_module(b)
+dist.init_process_group("gloo", rank=int(os.environ["RANK"]), world_size=2)
+b.DUMP_BYTES = 100 * 8 * 4
+y = torch.arange(1000, dtype=torch.float32)[:, None].repeat(1, 8)
+row0, row1 = (0, 640) if dist.get_rank() == 0 else (640, 1000)
+s = b.output_sample(y[row0:row1], 1000, row0, 2)
+if dist.get_rank() == 0:
+    print("SAMPLE", torch.equal(s, b.output_sample(y, 1000, 0, 1)), flush=True)
+dist.destroy_process_group()
+"""
+
+
+def test_output_sample_reassembles_the_row_shards_of_two_ranks(tmp_path):
+    import socket
+    s = socket.socket()
+    s.bind(("127.0.0.1", 0))
+    port = s.getsockname()[1]
+    s.close()
+    script = tmp_path / "sample.py"
+    script.write_text(_SAMPLE_SCRIPT)
+    procs = []
+    for r in range(2):
+        env = dict(os.environ, RANK=str(r), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), GLOO_SOCKET_IFNAME="lo")
+        procs.append(subprocess.Popen([sys.executable, str(script), os.path.join(ROOT, "bench.py")], env=env, stdout=subprocess.PIPE,
+                                      stderr=subprocess.PIPE, text=True))
+    outs = [p.communicate(timeout=120) for p in procs]
+    assert all(p.returncode == 0 for p in procs), [o[1][-500:] for o in outs]
+    assert "SAMPLE True" in outs[0][0]
 
 
 _LEAVE_SCRIPT = """

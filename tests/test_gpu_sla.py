@@ -6,15 +6,13 @@ Tolerances (the reference states none; SURVEY 8c):
   * attention output vs the fp32 block-sparse oracle on the same map: cosine >= 0.999, rel-L2 <= 2e-2;
     vs the INT8 emulation oracle: rel-L2 <= 1e-2.
 """
-import os
-
 import pytest
 import torch
 
+from oracle import golden
 from oracle import td_oracle as O
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _qkv(b, l, h, d, seed, kbias=2.0, dtype=torch.bfloat16):
@@ -93,7 +91,7 @@ def test_block_map_is_an_exact_topk_of_the_rounded_scores(cuda, b, l, h, d, rati
 def test_block_map_vs_reference_golden(cuda, name):
     """Golden from the reference's own get_block_map (torch.topk): equal as sets except at threshold ties."""
     from turbodiffusion_b200.SLA.utils import get_block_map
-    g = torch.load(os.path.join(GOLD, name + ".pt"))
+    g = golden.load(name)
     qh = g["q"].transpose(1, 2).contiguous().to(cuda)
     kh = g["k"].transpose(1, 2).contiguous().to(cuda)
     sparse_map, lut, topk = get_block_map(qh, kh, g["topk_ratio"], 128, 64)
@@ -167,7 +165,7 @@ def test_sage_sla_forward_vs_oracle(cuda, b, l, h, ratio):
 def test_sla_forward_vs_reference_golden(cuda, name):
     """End to end against the output of the reference's SparseLinearAttention.forward (Triton path, CPU interpreter)."""
     from turbodiffusion_b200.SLA import SparseLinearAttention
-    g = torch.load(os.path.join(GOLD, name + ".pt"))
+    g = golden.load(name)
     d = g["q"].shape[-1]
     mod = SparseLinearAttention(d, g["topk_ratio"], BLKQ=128, BLKK=64).to(cuda)
     with torch.no_grad():
@@ -235,7 +233,7 @@ def test_sage_sla_forward_head_dim_64_and_fp16(cuda, dtype):
 
 def test_sla_forward_vs_reference_golden_d64(cuda):
     from turbodiffusion_b200.SLA import SparseLinearAttention
-    g = torch.load(os.path.join(GOLD, "sla_b.pt"))
+    g = golden.load("sla_b")
     mod = SparseLinearAttention(64, g["topk_ratio"], BLKQ=128, BLKK=64).to(cuda)
     with torch.no_grad():
         mod.proj_l.weight.copy_(g["proj_w"])

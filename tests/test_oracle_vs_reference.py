@@ -5,13 +5,14 @@ import os
 import pytest
 import torch
 
+from oracle import golden
 from oracle import td_oracle as O
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _load(name):
-    return torch.load(os.path.join(GOLD, name + ".pt"))
+    return golden.load(name)
 
 
 def _max_ulp(got, ref):

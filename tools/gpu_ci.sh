@@ -11,7 +11,6 @@ for s in $STAGES; do
     slaprep) timeout 200 python -m pytest tests/test_gpu_sla.py -q -m gpu -k "quant_qk or block_map" > gpurun_out/t_slaprep.log 2>&1 ;;
     slamom) timeout 120 python -m pytest tests/test_gpu_sla.py -x -q -m gpu -k "linear_moments" > gpurun_out/t_slamom.log 2>&1 ;;
     slaattn) timeout 300 python -m pytest tests/test_gpu_sla.py -x -q -m gpu -k "forward" > gpurun_out/t_slaattn.log 2>&1 ;;
-    refext) timeout 300 python -m pytest tests/test_gpu_vs_reference_ext.py -q -m gpu -rs > gpurun_out/t_refext.log 2>&1 ;;
     mb)    timeout 400 python tools/microbench.py --iters 10 > gpurun_out/mb.log 2>&1 ;;
     bench) timeout 900 python bench.py > gpurun_out/bench.log 2>&1 ;;
     all)   timeout 1200 python -m pytest tests -x -q -m gpu > gpurun_out/t_all.log 2>&1 ;;
