@@ -165,7 +165,9 @@ int tdb200_rms_norm_rope_table(const void* x, int dtype, const float* w, const f
  *     sparse_map [b,h,mblk,nblk] int8 0/1 (SLA/utils.py:64-66) and lut [b,h,mblk,topk] int32 ascending block ids.
  * tdb200_sla_linear_moments   phi = softmax over d;  kv [b,h,d(v),d(k)] fp32 = sum_l v[l,:]^T phi(k)[l,:],
  *     ksum [b,h,d] fp32 = sum_l phi(k)[l,:]   (SLA/core.py:243-247).  Both must be zeroed by the caller
- *     (they are accumulated, so sequence shards can be summed with one all-reduce).
+ *     (they are accumulated, so sequence shards can be summed with one all-reduce).  These two entry points add the
+ *     partial sums of the CTAs that split l with fp32 atomics, in arrival order: the last bits vary from run to run.
+ *     tdb200_sla_linear_moments_ws is the bit-reproducible form.
  * tdb200_sla_attn_fwd   o = T( sparse_softmax_attention(q_i8,k_i8,v; lut) + proj( phi(q) kv / (1e-5 + phi(q).ksum) ) )
  *     kvw [b,h,d(out),d(k)] T = (proj_w . kv) so that proj is folded into the moment matrix; proj_b [d] fp32.
  *     The int8 QK^T, online softmax (exp2), PV, linear branch and merge run in one tcgen05 kernel.
@@ -181,6 +183,15 @@ int tdb200_sla_linear_moments(const void* k, const void* v, int dtype, int64_t b
  * 64 or 128 (kv [b,h,d,d], ksum [b,h,d]). */
 int tdb200_sla_linear_moments_ex(const void* k, const void* v, int dtype, int64_t b, int64_t l, int64_t h, int64_t d,
                                  int feature, float* kv, float* ksum, void* stream);
+/* Bit-reproducible moments: kv += sum, ksum += sum (same meaning and arguments as _ex), with the split-l partial sums
+ * stored to `workspace` and then reduced in a fixed order by a second kernel (2 launches).  The result depends on the inputs
+ * and the shape only: the same on every run and every device.  workspace: device memory of at least the size
+ * tdb200_sla_linear_moments_workspace reports for the shape (a host-side query, no CUDA call), 16-byte aligned, any
+ * contents, not read by the caller; ksum 16-byte aligned.  A smaller workspace returns TDB200_ERR_WORKSPACE.
+ * Calls that share one workspace must be ordered (the same stream). */
+int tdb200_sla_linear_moments_workspace(int64_t b, int64_t l, int64_t h, int64_t d, int64_t* bytes);
+int tdb200_sla_linear_moments_ws(const void* k, const void* v, int dtype, int64_t b, int64_t l, int64_t h, int64_t d,
+                                 int feature, float* kv, float* ksum, void* workspace, int64_t workspace_bytes, void* stream);
 /* kvw [bh,d,d] T = T(proj_w [d,d] . kv [bh,d,d]): folds proj_l's weight (SLA/core.py:246 `self.proj_l(o_l)`) into the moment
  * matrix so the fused kernel applies it with its last MMA; fp32 FMA chain over d_v. */
 int tdb200_sla_project_moments(const float* proj_w, const float* kv, int dtype, int64_t bh, int64_t d, void* kvw, void* stream);

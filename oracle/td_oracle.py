@@ -499,10 +499,12 @@ def ltx_gemm_post_scale(a_q, a_s, b_q, b_s, bias, out_dtype=torch.bfloat16) -> t
 # One Wan DiT block's self-attention + FFN hot path (for bench cpu_baseline / block parity), wan2pt1.py:390-417
 # =============================================================================================
 def wan_block_forward(sd: dict, x: torch.Tensor, e0: torch.Tensor, angles: torch.Tensor, context: torch.Tensor,
-                      dim: int, heads: int, eps: float = 1e-6, topk: float = 0.1, sla_mode: str = "exact") -> torch.Tensor:
+                      dim: int, heads: int, eps: float = 1e-6, topk: float = 0.1, sla_mode: str = "exact",
+                      lut: Optional[torch.Tensor] = None) -> torch.Tensor:
     """WanAttentionBlock.forward (rcm/networks/wan2pt1.py:390-417) after TurboDiffusion's model surgery
     (inference/modify_model.py:40-81), on CPU tensors.  `sd`: reference state-dict keys relative to blocks.<i>.
-    x [L, dim], e0 [6, dim] fp32, angles [L, head_dim/2], context [Lc, dim]."""
+    x [L, dim], e0 [6, dim] fp32, angles [L, head_dim/2], context [Lc, dim].  `lut` [1, heads, Mblk, topk]: the key blocks
+    the self-attention attends to (default: the oracle's own top-k selection)."""
     d = dim // heads
     l = x.shape[0]
 
@@ -517,7 +519,7 @@ def wan_block_forward(sd: dict, x: torch.Tensor, e0: torch.Tensor, angles: torch
     v = lin(hmod, "self_attn.v").view(l, heads, d)
     q, k = rope_interleaved(q, angles), rope_interleaved(k, angles)
     a = sla_forward(q[None], k[None], v[None], sd["self_attn.attn_op.local_attn.proj_l.weight"],
-                    sd["self_attn.attn_op.local_attn.proj_l.bias"], topk, mode=sla_mode)[0].reshape(l, dim)
+                    sd["self_attn.attn_op.local_attn.proj_l.bias"], topk, mode=sla_mode, lut=lut)[0].reshape(l, dim)
     x = gate_residual(x, lin(a, "self_attn.o"), e[2])
     hn = fast_layernorm(x, sd["norm3.weight"], sd["norm3.bias"], eps)
     cq = fast_rmsnorm(lin(hn, "cross_attn.q"), sd["cross_attn.norm_q.weight"], eps).view(1, l, heads, d)

@@ -79,7 +79,7 @@ def test_argument_validation_of_every_kernel_family(libpath):
     (never exit(), never a crash), so the contract can be exercised on a machine without a GPU."""
     from turbodiffusion_b200 import _lib
     lib = _lib.lib()
-    INVALID, UNSUPPORTED = -1, -2
+    INVALID, UNSUPPORTED, WORKSPACE = -1, -2, -5
     cases = [
         ("quant null", lambda: lib.tdb200_quant_int8_block128(None, 0, 128, 128, _p(), _p(), None), INVALID, b"null"),
         ("gemm k%128", lambda: lib.tdb200_gemm_w8a8(_p(), _p(), _p(), _p(), None, _p(), 0, 128, 128, 100, None), UNSUPPORTED, b"128"),
@@ -93,6 +93,16 @@ def test_argument_validation_of_every_kernel_family(libpath):
         ("block map topk", lambda: lib.tdb200_sla_block_map(_p(), _p(), 0, 1, 2, 4, 8, 128, 9, _p(), _p(), None), INVALID, b"topk"),
         ("moments head dim", lambda: lib.tdb200_sla_linear_moments(_p(), _p(), 0, 1, 256, 2, 96, _p(), _p(), None), UNSUPPORTED, b"head dim"),
         ("moments feature map", lambda: lib.tdb200_sla_linear_moments_ex(_p(), _p(), 0, 1, 256, 2, 64, 7, _p(), _p(), None), INVALID, b"feature"),
+        ("moments ws too small", lambda: lib.tdb200_sla_linear_moments_ws(_p(), _p(), 0, 1, 256, 2, 128, 0, _p(), _p(), _p(), 1024, None),
+         WORKSPACE, b"needed"),
+        ("moments ws null", lambda: lib.tdb200_sla_linear_moments_ws(_p(), _p(), 0, 1, 256, 2, 128, 0, _p(), _p(), None, 1 << 30, None),
+         INVALID, b"null"),
+        ("moments ws head dim", lambda: lib.tdb200_sla_linear_moments_ws(_p(), _p(), 0, 1, 256, 2, 96, 0, _p(), _p(), _p(), 1 << 30, None),
+         UNSUPPORTED, b"head dim"),
+        ("moments ws ksum misaligned", lambda: lib.tdb200_sla_linear_moments_ws(_p(), _p(), 0, 1, 256, 2, 128, 0, _p(), _p(4100), _p(),
+                                                                                 1 << 30, None), INVALID, b"aligned"),
+        ("moments workspace shape", lambda: lib.tdb200_sla_linear_moments_workspace(0, 256, 2, 128, ctypes.byref(ctypes.c_int64())),
+         INVALID, b"shape"),
         ("attn v2 head dim", lambda: lib.tdb200_sla_attn_fwd_v2(_p(), _p(), _p(), _p(), _p(), _p(), 0, _p(), 4, _p(), _p(), _p(), _p(), 1, 256,
                                                                 256, 2, 96, 0.088, 0, None), UNSUPPORTED, b"head dim"),
         ("gelu quant k", lambda: lib.tdb200_gelu_quant_int8_block128(_p(), 0, 128, 100, _p(), _p(), None), UNSUPPORTED, b"multiple of 8"),
@@ -116,6 +126,27 @@ def test_argument_validation_of_every_kernel_family(libpath):
         msg = lib.tdb200_last_error() or b""
         assert rc == code, (name, rc, msg)
         assert needle in msg, (name, msg)
+
+
+def test_moments_workspace_size_is_a_function_of_the_shape(libpath):
+    """The size query runs on the host: splits = min(tiles, max(1, 148 // (b * head units))) slots of kv [b,h,d,d] + ksum
+    [b,h,d] fp32; 64-wide heads are paired into one unit."""
+    from turbodiffusion_b200 import _lib
+    lib = _lib.lib()
+
+    def size(b, l, h, d):
+        n = ctypes.c_int64(-1)
+        assert lib.tdb200_sla_linear_moments_workspace(b, l, h, d, ctypes.byref(n)) == 0, lib.tdb200_last_error()
+        return n.value
+
+    assert size(1, 32760, 12, 128) == 12 * 12 * 128 * 129 * 4      # shape A: 12 splits of the 256 key tiles
+    assert size(1, 75600, 40, 128) == 3 * 40 * 128 * 129 * 4       # 14B: 3 splits
+    assert size(1, 32760, 24, 64) == 12 * 24 * 64 * 65 * 4         # 12 pairs of 64-wide heads
+    assert size(1, 32760, 23, 64) == 12 * 23 * 64 * 65 * 4         # an odd head count: the last pair is half empty
+    assert size(1, 200, 2, 128) == 2 * 2 * 128 * 129 * 4            # no more splits than 128-row tiles
+    assert size(4, 1000, 40, 128) == 1 * 4 * 40 * 128 * 129 * 4     # more head units than SMs: one split
+    rc = lib.tdb200_sla_linear_moments_ws(_p(), _p(), 0, 1, 32760, 12, 128, 0, _p(), _p(), _p(), size(1, 32760, 12, 128) - 16, None)
+    assert rc == -5 and b"needed" in lib.tdb200_last_error()
 
 
 def test_valid_calls_without_a_gpu_report_an_error_code(libpath):

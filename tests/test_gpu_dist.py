@@ -56,7 +56,7 @@ def test_sequence_parallel_matches_single_gpu(tmp_path, mode, dim, heads):
     out = str(tmp_path / "sp.pt")
     mp.spawn(_worker, args=(2, port, out, mode, dim, heads), nprocs=2, join=True)
     res = torch.load(out)
-    # identical arithmetic per row; only the fp32 summation order of the linear-attention moments differs (atomics, and the
-    # all-reduce in the all-gather mode), which moves the 16-bit kvw operand and through it many outputs by one unit in the
+    # identical arithmetic per row; only the fp32 summation order of the linear-attention moments differs (per-rank partial
+    # sums, and the all-reduce in the all-gather mode), which moves the 16-bit kvw operand and through it many outputs by one unit in the
     # last place: measured 1e-3 .. 2.4e-3 (uneven-head split) with max |diff| = 1 bf16 ulp of the largest outputs
     assert res["rel_l2"] < 4e-3 and res["max_abs"] <= 0.0625, res

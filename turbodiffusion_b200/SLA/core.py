@@ -3,12 +3,15 @@
 Same constructor arguments, parameters (`proj_l`, fp32, zero-init) and call convention (q,k,v in [B, L, H, D], result in
 the same layout and dtype; SLA/core.py:181-183,253).  The forward is five kernel launches:
   quant_qk (key mean, pooled means, INT8 Q / smoothed K)  ->  block_map (pooled score, top-k, LUT)
-  -> linear_moments (phi(K)^T V, sum phi(K))  ->  [tiny cuBLAS bmm: proj_l folded into the moment matrix]
+  -> linear_moments (phi(K)^T V, sum phi(K); split-L partials reduced in a fixed order)  ->  project_moments (proj_l folded
+  into the moment matrix)
   -> attn_fwd (sparse INT8 QK^T, softmax, PV, linear branch, merge).
 Inputs are consumed in place in their [B, L, H, D] layout; no transposed copies of q/k/v are made.
 """
 from __future__ import annotations
 
+import ctypes
+import functools
 import os
 
 import torch
@@ -25,14 +28,25 @@ SAGE2PP_ENABLED = True
 FEATURE_TAG = {"softmax": 0, "elu": 1, "relu": 2}   # SLA/core.py:57-73
 
 
+@functools.lru_cache(maxsize=256)
+def moments_workspace_bytes(b: int, l: int, h: int, d: int) -> int:
+    """Scratch bytes tdb200_sla_linear_moments_ws needs for k/v [b, l, h, d] (a function of the shape alone)."""
+    n = ctypes.c_int64(0)
+    check(lib().tdb200_sla_linear_moments_workspace(b, l, h, d, ctypes.byref(n)), "sla_linear_moments_workspace", launches=0)
+    return n.value
+
+
 def linear_moments(k: torch.Tensor, v: torch.Tensor, feature: int = 0):
     """kv [B,H,D(v),D(k)] fp32, ksum [B,H,D] fp32 of the local keys (accumulated: add shards / all-reduce).  D in {64, 128};
-    `feature`: 0 softmax over D, 1 elu+1, 2 relu."""
+    `feature`: 0 softmax over D, 1 elu+1, 2 relu.  Bit-reproducible: the partial sums of the CTAs that split L are reduced
+    in a fixed order."""
     b, l, h, d = k.shape
     buf = torch.zeros(b * h * d * (d + 1), dtype=torch.float32, device=k.device)        # one fill for both accumulators
     kv, ksum = buf[: b * h * d * d].view(b, h, d, d), buf[b * h * d * d:].view(b, h, d)
-    check(lib().tdb200_sla_linear_moments_ex(ptr(k), ptr(v), DTYPE_TAG[k.dtype], b, l, h, d, feature, ptr(kv), ptr(ksum),
-                                             stream_ptr(k.device)), "sla_linear_moments")
+    nbytes = moments_workspace_bytes(b, l, h, d)
+    ws = torch.empty(nbytes // 4, dtype=torch.float32, device=k.device)
+    check(lib().tdb200_sla_linear_moments_ws(ptr(k), ptr(v), DTYPE_TAG[k.dtype], b, l, h, d, feature, ptr(kv), ptr(ksum),
+                                             ptr(ws), nbytes, stream_ptr(k.device)), "sla_linear_moments")
     return kv, ksum
 
 

@@ -45,6 +45,8 @@ _PROTOS = {
     "tdb200_sla_block_map": [_P, _P, _I, _I64, _I64, _I64, _I64, _I64, _I64, _P, _P, _P],
     "tdb200_sla_linear_moments": [_P, _P, _I, _I64, _I64, _I64, _I64, _P, _P, _P],
     "tdb200_sla_linear_moments_ex": [_P, _P, _I, _I64, _I64, _I64, _I64, _I, _P, _P, _P],
+    "tdb200_sla_linear_moments_workspace": [_I64, _I64, _I64, _I64, ctypes.POINTER(c_int64)],
+    "tdb200_sla_linear_moments_ws": [_P, _P, _I, _I64, _I64, _I64, _I64, _I, _P, _P, _P, _I64, _P],
     "tdb200_sla_attn_fwd": [_P, _P, _P, _P, _P, _P, _I, _P, _I64, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _I64, _F,
                             _P],
     "tdb200_sla_attn_fwd_kseq": [_P, _P, _P, _P, _P, _P, _I, _P, _I64, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _I64, _F,
@@ -130,7 +132,7 @@ class _DeviceGuarded:
 
 
 LAUNCHES = 0  # kernels launched through the C ABI (each entry point documents how many it enqueues)
-_KERNELS_PER_CALL = {"sla_quant_qk": 4, "layernorm_modulate_quant": 2}  # upper bounds per entry point
+_KERNELS_PER_CALL = {"sla_quant_qk": 4, "layernorm_modulate_quant": 2, "sla_linear_moments": 2}  # upper bounds per entry point
 
 
 def check(rc: int, what: str, launches: int = None) -> None:

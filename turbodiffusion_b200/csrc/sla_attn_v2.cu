@@ -411,7 +411,10 @@ sla_attn_v2_kernel(const __grid_constant__ CUtensorMap tmap_q8, const __grid_con
             pw[hc * 8 + (c >> 1) + 1] = F16Traits<T>::pack(t1.x, t1.y);
           }
         }
-        tc_fence_before_sync();                            // my tcgen05.ld of S precede the partner's P store into S
+        // P(j) of half hf goes to columns [16*hf, 16*hf+16) of this S buffer: half 1 stores over S columns [16, 32), which
+        // half 0 reads in pass 2.  Both halves finish reading S before either stores P.
+        tc_fence_before_sync();
+        named_bar_sync(pair_bar, 64);
         const float2 ps2 = __fadd2_rn(psa, psb);
         float psum = ps2.x + ps2.y;
         if (valid < 32) {

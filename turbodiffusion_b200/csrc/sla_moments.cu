@@ -2,8 +2,14 @@
 //   phi = softmax over the head dim (rounded to the 16-bit type),
 //   kv[b,h,dv,dk] += sum_l v[l,dv] * phi(k)[l,dk]        (stored transposed: rows = value channel, cols = key channel)
 //   ksum[b,h,dk]  += sum_l phi(k)[l,dk]
-// Both outputs are ACCUMULATED in fp32 with red.global.add (caller zeroes them), so sequence shards and the split-L
-// CTAs of one GPU combine by plain addition (and one all-reduce across GPUs).
+// Both outputs are ACCUMULATED (caller zeroes them), so sequence shards combine by plain addition (one all-reduce across
+// GPUs).  The L axis of one head is split over `splits` CTAs.  tdb200_sla_linear_moments_ws combines the split partials in a
+// fixed order: every CTA stores its partial to a workspace slot, then a second kernel sums the slots in ascending split order
+// and adds the sum once (bit-reproducible).  The workspace entry points fix `splits` from the shape alone (kSplitTarget), so
+// the result does not depend on the SM count either.  The older entry points add the partials with fp32 red.global.add in
+// arrival order instead (the last bits of kv / ksum then vary from run to run).
+// A second kernel rather than a last-CTA-reduces ticket: no counter state that must be zero before the call, and the
+// ~0.8 MB of partials per head at shape A are summed by the whole GPU instead of by one SM at the tail of the kernel.
 //
 // CTA = 6 warps, 128 key rows per tile.  warps 0-3: thread == key row: load the row, softmax over D (MUFU ex2), write
 // phi(k) into shared memory in the MN-major 128B-swizzled operand layout, then column-sum the tile for ksum.
@@ -39,6 +45,9 @@ struct MomParams {
   const void* k;
   float* kv;
   float* ksum;
+  float* part;   // NULL: red.global.add into kv / ksum; else split s stores its partial to part + s * slot (plain stores)
+  int64_t slot;  // floats per workspace slot: kv [b,h,hd,hd] at offset 0, then ksum [b,h,hd] at offset kv_elems
+  int64_t kv_elems;
   int l, h, tiles, splits;
   int hd;        // 128, or 64 (two heads per 128-wide row; `h` is then the number of REAL heads, grid.x = ceil(h/2) pairs)
   int feature;   // 0 softmax, 1 elu+1, 2 relu
@@ -46,6 +55,19 @@ struct MomParams {
 
 __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+}
+
+// accumulate into kv / ksum (atomic) or store into this CTA's own workspace slot (plain)
+__device__ __forceinline__ void put_v4(bool plain, float* addr, const uint32_t* o) {
+  if (plain)
+    *reinterpret_cast<float4*>(addr) = make_float4(__uint_as_float(o[0]), __uint_as_float(o[1]), __uint_as_float(o[2]),
+                                                   __uint_as_float(o[3]));
+  else
+    red_add_v4(addr, __uint_as_float(o[0]), __uint_as_float(o[1]), __uint_as_float(o[2]), __uint_as_float(o[3]));
+}
+__device__ __forceinline__ void put_f32(bool plain, float* addr, float x) {
+  if (plain) *addr = x;
+  else atomicAdd(addr, x);
 }
 
 template <typename T, bool kPair>
@@ -62,6 +84,9 @@ sla_moments_kernel(const __grid_constant__ CUtensorMap tmap_v, MomParams p) {
   const bool second_ok = !pair || head0 + 1 < p.h;                 // odd head count: the last pair has one real head
   const int64_t row_elems = int64_t(p.h) * p.hd;                   // elements per token row of k / v
   const int my_tiles = (p.tiles - split + p.splits - 1) / p.splits;  // tiles split, split+splits, ...
+  const bool plain = p.part != nullptr;
+  float* const kv_out = plain ? p.part + split * p.slot : p.kv;
+  float* const ksum_out = plain ? p.part + split * p.slot + p.kv_elems : p.ksum;
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < 2; ++i) {
@@ -77,7 +102,7 @@ sla_moments_kernel(const __grid_constant__ CUtensorMap tmap_v, MomParams p) {
   __syncthreads();
   tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_slot;
-  if (my_tiles <= 0) {  // nothing to do (more splits than tiles); still release TMEM
+  if (my_tiles <= 0) {  // nothing to do (more splits than tiles; the host clamps splits <= tiles); still release TMEM
     __syncthreads();
     if (warp == 5) tmem_dealloc<128>(tmem_base);
     return;
@@ -219,29 +244,27 @@ sla_moments_kernel(const __grid_constant__ CUtensorMap tmap_v, MomParams p) {
     }
     // thread r holds key channel r of the 128-wide row: head0's channel r, or (pairs) channel r-64 of head0+1
     if (!pair) {
-      atomicAdd(p.ksum + (int64_t(b) * p.h + head0) * D + r, ksum_acc);
+      put_f32(plain, ksum_out + (int64_t(b) * p.h + head0) * D + r, ksum_acc);
     } else if (r < 64 || second_ok) {
-      atomicAdd(p.ksum + (int64_t(b) * p.h + head0 + (r >> 6)) * 64 + (r & 63), ksum_acc);
+      put_f32(plain, ksum_out + (int64_t(b) * p.h + head0 + (r >> 6)) * 64 + (r & 63), ksum_acc);
     }
     // ---- kv: TMEM lane r = value channel r, 128 key channels
     mbar_wait(&bars[kAccFull], 0);
     tc_fence_after_sync();
     if (!pair) {
-      float* dst = p.kv + ((int64_t(b) * p.h + head0) * D + r) * D;
+      float* dst = kv_out + ((int64_t(b) * p.h + head0) * D + r) * D;
 #pragma unroll
       for (int c = 0; c < D / 32; ++c) {
         uint32_t o[32];
         tmem_ld_x32(tmem_base + (uint32_t(warp * 32) << 16) + c * 32, o);
         tmem_ld_wait();
 #pragma unroll
-        for (int q = 0; q < 32; q += 4)
-          red_add_v4(dst + c * 32 + q, __uint_as_float(o[q]), __uint_as_float(o[q + 1]), __uint_as_float(o[q + 2]),
-                     __uint_as_float(o[q + 3]));
+        for (int q = 0; q < 32; q += 4) put_v4(plain, dst + c * 32 + q, o + q);
       }
     } else {
       // lane r = value channel (r & 63) of head0 + (r >> 6); its diagonal block is key columns [64*(r>>6), +64)
       const int sub = r >> 6;                        // warp-uniform (warps 0,1 -> head0; warps 2,3 -> head0+1)
-      float* dst = p.kv + ((int64_t(b) * p.h + head0 + sub) * 64 + (r & 63)) * 64;
+      float* dst = kv_out + ((int64_t(b) * p.h + head0 + sub) * 64 + (r & 63)) * 64;
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
         uint32_t o[32];
@@ -249,9 +272,7 @@ sla_moments_kernel(const __grid_constant__ CUtensorMap tmap_v, MomParams p) {
         tmem_ld_wait();
         if (sub == 0 || second_ok) {
 #pragma unroll
-          for (int q = 0; q < 32; q += 4)
-            red_add_v4(dst + c * 32 + q, __uint_as_float(o[q]), __uint_as_float(o[q + 1]), __uint_as_float(o[q + 2]),
-                       __uint_as_float(o[q + 3]));
+          for (int q = 0; q < 32; q += 4) put_v4(plain, dst + c * 32 + q, o + q);
         }
       }
     }
@@ -264,17 +285,54 @@ sla_moments_kernel(const __grid_constant__ CUtensorMap tmap_v, MomParams p) {
   }
 }
 
-}  // namespace
+// kv += sum_s part[s][0, kv_elems), ksum += sum_s part[s][kv_elems, slot): one float4 per thread, splits summed in
+// ascending order in fp32, then added to the accumulator once.
+__global__ void __launch_bounds__(256) moments_reduce_kernel(const float4* __restrict__ part, float4* kv, float4* ksum,
+                                                              int64_t kv4, int64_t slot4, int splits) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= slot4) return;
+  float4 acc = part[i];
+  for (int s = 1; s < splits; ++s) {
+    const float4 x = part[s * slot4 + i];
+    acc.x += x.x; acc.y += x.y; acc.z += x.z; acc.w += x.w;
+  }
+  float4* dst = i < kv4 ? kv + i : ksum + (i - kv4);
+  float4 y = *dst;
+  y.x += acc.x; y.y += acc.y; y.z += acc.z; y.w += acc.w;
+  *dst = y;
+}
 
-static int moments_impl(const void* k, const void* v, int dtype, int64_t b, int64_t l, int64_t h, int64_t d, int feature,
-                        float* kv, float* ksum, void* stream) {
-  using namespace tdb;
+// CTAs per head unit for the workspace entry points: one wave of a 148-SM B200 at b * units <= 148, a function of the shape
+// only (the workspace size is then known without a device, and the summation order is the same on every GPU).
+constexpr int kSplitTarget = 148;
+
+int64_t units_of(int64_t h, int64_t d) { return d == 128 ? h : cdiv64(h, 2); }  // CTAs along x: heads, or pairs of 64-wide heads
+
+int splits_of(int64_t sms, int64_t b, int64_t l, int64_t h, int64_t d) {
+  const int64_t tiles = cdiv64(l, kRowsPerTile);
+  int64_t splits = sms / (b * units_of(h, d));
+  if (splits < 1) splits = 1;
+  if (splits > tiles) splits = tiles;
+  return int(splits);
+}
+
+int check_shape(const void* k, const void* v, int64_t b, int64_t l, int64_t h, int64_t d, int feature, float* kv, float* ksum) {
   if (!k || !v || !kv || !ksum) return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments: null pointer");
-  if (b <= 0 || l <= 0 || h <= 0) return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments: bad shape");
+  if (b <= 0 || l <= 0 || h <= 0 || l > 0x7FFFFFFF) return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments: bad shape");
   if (d != 64 && d != 128) return fail(TDB200_ERR_UNSUPPORTED, "sla_linear_moments: head dim %lld (64 or 128, SLA/core.py:207)", (long long)d);
   if (feature < 0 || feature > 2) return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments: feature map tag %d", feature);
   if (h > 65535 || b > 65535) return fail(TDB200_ERR_UNSUPPORTED, "sla_linear_moments: h or b too large");
   if (!aligned16(k) || !aligned16(kv)) return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments: buffers must be 16-byte aligned");
+  return TDB200_OK;
+}
+
+}  // namespace
+
+// part == NULL: the split partials are added into kv / ksum with fp32 atomics (order of arrival).  Otherwise part holds
+// `splits` slots of MomParams::slot floats and a second kernel reduces them in a fixed order.
+static int moments_impl(const void* k, const void* v, int dtype, int64_t b, int64_t l, int64_t h, int64_t d, int feature,
+                        float* kv, float* ksum, float* part, int splits, void* stream) {
+  using namespace tdb;
   if (int rc = require_sm100()) return rc;
   const CUtensorMapDataType t16 = dtype == TDB200_DTYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
   CUtensorMap tv;
@@ -284,47 +342,81 @@ static int moments_impl(const void* k, const void* v, int dtype, int64_t b, int6
     const uint32_t box[4] = {64, 1, kRowsPerTile, 1};
     if (int rc = make_tmap_4d(&tv, v, t16, 2, dims, str, box)) return rc;
   }
-  const int64_t units = d == 128 ? h : cdiv64(h, 2);   // CTAs along x: heads, or pairs of 64-wide heads
   MomParams p;
   p.k = k;
   p.kv = kv;
   p.ksum = ksum;
+  p.part = part;
+  p.kv_elems = b * h * d * d;
+  p.slot = p.kv_elems + b * h * d;
   p.l = int(l);
   p.h = int(h);
   p.hd = int(d);
   p.feature = feature;
   p.tiles = int(cdiv64(l, kRowsPerTile));
-  int splits = sm_count() / int(b * units);
-  if (splits < 1) splits = 1;
-  if (splits > p.tiles) splits = p.tiles;
   p.splits = splits;
-  dim3 grid(static_cast<unsigned>(units), splits, static_cast<unsigned>(b));
+  dim3 grid(static_cast<unsigned>(units_of(h, d)), splits, static_cast<unsigned>(b));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = TDB200_OK;
 #define TDB_MOM2(T, PAIR)                                                                                          \
   do {                                                                                                              \
     static bool attr_done[64] = {false};                                                                            \
-    if (int rc = set_max_dynamic_smem_once(reinterpret_cast<const void*>(sla_moments_kernel<T, PAIR>), kSmemBytes, attr_done, \
-                                           "cudaFuncSetAttribute(sla_moments)"))                                   \
-      return rc;                                                                                                    \
+    if (int e = set_max_dynamic_smem_once(reinterpret_cast<const void*>(sla_moments_kernel<T, PAIR>), kSmemBytes, attr_done, \
+                                          "cudaFuncSetAttribute(sla_moments)"))                                    \
+      return e;                                                                                                     \
     sla_moments_kernel<T, PAIR><<<grid, kThreads, kSmemBytes, st>>>(tv, p);                                         \
-    return check_launch("sla_moments_kernel");                                                                      \
+    rc = check_launch("sla_moments_kernel");                                                                        \
   } while (0)
 #define TDB_MOM(T) do { if (d == 64) { TDB_MOM2(T, true); } else { TDB_MOM2(T, false); } } while (0)
   if (dtype == TDB200_DTYPE_BF16) TDB_MOM(__nv_bfloat16);
-  if (dtype == TDB200_DTYPE_FP16) TDB_MOM(__half);
+  else if (dtype == TDB200_DTYPE_FP16) TDB_MOM(__half);
+  else return fail(TDB200_ERR_UNSUPPORTED, "sla_linear_moments: dtype tag %d", dtype);
 #undef TDB_MOM2
 #undef TDB_MOM
-  return fail(TDB200_ERR_UNSUPPORTED, "sla_linear_moments: dtype tag %d", dtype);
+  if (rc != TDB200_OK || part == nullptr) return rc;
+  const int64_t slot4 = p.slot / 4;   // kv_elems and slot are multiples of 4 (d * d and d are)
+  moments_reduce_kernel<<<static_cast<unsigned>(cdiv64(slot4, 256)), 256, 0, st>>>(
+      reinterpret_cast<const float4*>(part), reinterpret_cast<float4*>(kv), reinterpret_cast<float4*>(ksum), p.kv_elems / 4,
+      slot4, splits);
+  return check_launch("moments_reduce_kernel");
 }
 
 extern "C" int tdb200_sla_linear_moments(const void* k, const void* v, int dtype, int64_t b, int64_t l, int64_t h,
                                          int64_t d, float* kv, float* ksum, void* stream) {
-  return moments_impl(k, v, dtype, b, l, h, d, 0, kv, ksum, stream);
+  return tdb200_sla_linear_moments_ex(k, v, dtype, b, l, h, d, 0, kv, ksum, stream);
 }
 
 extern "C" int tdb200_sla_linear_moments_ex(const void* k, const void* v, int dtype, int64_t b, int64_t l, int64_t h,
                                             int64_t d, int feature, float* kv, float* ksum, void* stream) {
-  return moments_impl(k, v, dtype, b, l, h, d, feature, kv, ksum, stream);
+  if (int rc = check_shape(k, v, b, l, h, d, feature, kv, ksum)) return rc;
+  return moments_impl(k, v, dtype, b, l, h, d, feature, kv, ksum, nullptr, splits_of(tdb::sm_count(), b, l, h, d), stream);
+}
+
+extern "C" int tdb200_sla_linear_moments_workspace(int64_t b, int64_t l, int64_t h, int64_t d, int64_t* bytes) {
+  using namespace tdb;
+  if (!bytes) return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments_workspace: null pointer");
+  if (b <= 0 || l <= 0 || h <= 0 || l > 0x7FFFFFFF || h > 65535 || b > 65535)
+    return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments_workspace: bad shape");
+  if (d != 64 && d != 128) return fail(TDB200_ERR_UNSUPPORTED, "sla_linear_moments_workspace: head dim %lld (64 or 128)", (long long)d);
+  *bytes = int64_t(splits_of(kSplitTarget, b, l, h, d)) * (b * h * d * (d + 1)) * int64_t(sizeof(float));
+  return TDB200_OK;
+}
+
+extern "C" int tdb200_sla_linear_moments_ws(const void* k, const void* v, int dtype, int64_t b, int64_t l, int64_t h,
+                                            int64_t d, int feature, float* kv, float* ksum, void* workspace,
+                                            int64_t workspace_bytes, void* stream) {
+  using namespace tdb;
+  if (int rc = check_shape(k, v, b, l, h, d, feature, kv, ksum)) return rc;
+  if (!workspace) return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments_ws: null workspace");
+  if (!aligned16(ksum) || !aligned16(workspace))
+    return fail(TDB200_ERR_INVALID_ARG, "sla_linear_moments_ws: ksum and workspace must be 16-byte aligned");
+  int64_t need = 0;
+  if (int rc = tdb200_sla_linear_moments_workspace(b, l, h, d, &need)) return rc;
+  if (workspace_bytes < need)
+    return fail(TDB200_ERR_WORKSPACE, "sla_linear_moments_ws: workspace of %lld bytes, %lld needed", (long long)workspace_bytes,
+                (long long)need);
+  return moments_impl(k, v, dtype, b, l, h, d, feature, kv, ksum, static_cast<float*>(workspace),
+                      splits_of(kSplitTarget, b, l, h, d), stream);
 }
 
 // ---- kvw = T(proj_w . kv): the linear branch's output projection folded into the moment matrix (SLA/core.py:243-253:
